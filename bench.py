@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- TPC-H Q1/Q6/Q3 lineitem rows/s + HBM roofline fraction at SF100 on N B200s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--sf 100] [--queries q6,q1,q3]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--sf 100] [--queries q6,q1,q3] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...      # the reference's CPU path (oracle port) on host cores
 
@@ -44,7 +44,15 @@ def parse_args():
     ap.add_argument("--no-chunked-e2e", action="store_true", help="skip the 2048-row-chunk pageable-memory e2e leg (C++ host shim subprocess)")
     ap.add_argument("--cpu-sample-sf", type=float, default=None,
                     help="CPU sample: this SF worth of rows (default: 4 for the cpu_baseline leg, 10 for --impl reference, shrunk to fit the time bound)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result columns of the last timed step as DIR/<query>_col<i>.npy (float64), so that two builds "
+                         "can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
+    return args
 
 
 def measured_peak_gbs():
@@ -131,6 +139,56 @@ def parity_check(X, q, chunks, sf):
         return None
     order, ncols = PARITY_RENDER[q]
     return X.rows_text(X.order_limit(chunks, order), ncols) == open(fx).read()
+
+
+# ----------------------------------------------------------------------------------------
+# --dump-outputs: the result columns of the last timed step, as numbers
+# ----------------------------------------------------------------------------------------
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def column_values(vec):
+    """One result vector as float64: DECIMAL / HUGEINT records as their numeric value, codes of CHAR / DICT columns as
+    numbers, NULL as NaN."""
+    import numpy as np
+    d = vec.Data
+    if d.dtype.names == ("coef", "scale", "neg"):
+        x = d["coef"].astype(np.float64) / 10.0 ** d["scale"].astype(np.float64)
+        x = np.where(d["neg"] != 0, -x, x)
+    elif d.dtype.names == ("lower", "upper"):
+        x = d["upper"].astype(np.float64) * 2.0 ** 64 + d["lower"].astype(np.float64)
+    else:
+        x = d.astype(np.float64)
+    if vec.Mask is not None:
+        valid = np.unpackbits(vec.Mask, bitorder="little")[:len(x)].astype(bool)
+        x = np.where(valid, x, np.nan)
+    return x
+
+
+def dump_outputs(path, results):
+    """results: {query: (chunks, number of result columns)}.  Rows are put in the order of the host ORDER BY that stays in
+    Go (PARITY_RENDER), so that the files do not depend on the order in which the device emitted groups.  Above
+    DUMP_LIMIT_BYTES in all, every query keeps the same fixed, seeded sample fraction of its rows."""
+    import numpy as np
+    cols = {}
+    for q, (chunks, ncols) in results.items():
+        qc = [np.concatenate([column_values(c.Data[i]) for c in chunks]) if chunks else np.zeros(0) for i in range(ncols)]
+        order = PARITY_RENDER.get(q, ([], 0))[0]
+        if order and qc and len(qc[0]):
+            idx = np.lexsort([-qc[i] if desc else qc[i] for i, desc in reversed(order)])
+            qc = [c[idx] for c in qc]
+        cols[q] = qc
+    total = sum(c.nbytes for qc in cols.values() for c in qc)
+    rng = np.random.default_rng(0)
+    os.makedirs(path, exist_ok=True)
+    for q, qc in cols.items():
+        n = len(qc[0]) if qc else 0
+        if total > DUMP_LIMIT_BYTES:
+            keep = np.sort(rng.choice(n, n * DUMP_LIMIT_BYTES // total, replace=False))
+            qc = [c[keep] for c in qc]
+        for i, c in enumerate(qc):
+            np.save(os.path.join(path, "%s_col%d.npy" % (q, i)), c)
 
 
 # ----------------------------------------------------------------------------------------
@@ -291,8 +349,10 @@ def main():
         return chunks, ex.stats
 
     def step(acc=None):
+        results = {}
         for q in queries:
-            _, st = run_query(q)
+            chunks, st = run_query(q)
+            results[q] = chunks
             if acc is not None:
                 a = acc.setdefault(q, {"kernel_ms": 0.0, "main_ms": 0.0, "exec_ms": 0.0, "launches": 0, "n": 0,
                                        "bytes": st.algorithmic_bytes, "main_bytes": st.main_kernel_bytes})
@@ -301,6 +361,7 @@ def main():
                 a["exec_ms"] += st.exec_ms
                 a["launches"] += st.kernel_launches
                 a["n"] += 1
+        return results
 
     sampler = ClockSampler(local_rank)
     if rank == 0:
@@ -314,7 +375,7 @@ def main():
     barrier()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step(acc)
+        last = step(acc)
     barrier()
     dt = max_over_ranks(time.perf_counter() - t0)
     # the timed region can be a few milliseconds: keep the same steps running (untimed) until the
@@ -327,6 +388,8 @@ def main():
         clocks["note"] = "sampled every 100 ms from warm-up through the timed steps and 0.6 s of the same steps after"
     ms_per_step = dt / args.steps * 1e3
     value = total_rows * len(queries) * args.steps / dt
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {q: (last[q], len(execs[q].coltypes)) for q in queries})
 
     # ---- parity (untimed): the results of THIS run, on every rank, against the committed fixtures --------
     def all_ranks_agree(flag):

@@ -1,5 +1,5 @@
-import sys, time, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, time, numpy as np, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from plan_b200 import _lib as L, compute as X, tpch as T, chunk as K
 sf = float(sys.argv[1])
 lib = L.lib(); L.check(lib.pg_init(0))
