@@ -1343,6 +1343,7 @@ struct JoinAggPipeline : Pipeline {
             ngroups = (i64)ng2[0];
             dense_passes = npass;
         }
+        bool op_crowded = false;         // the order-preserving map overflowed: keys crowd a few home slots
         for (int attempt = 0; !sorted_runs && !dense_group; attempt++) {
             PG_TRY(ensure_group_table(cap));
             cap = gt_cap;
@@ -1355,7 +1356,7 @@ struct JoinAggPipeline : Pipeline {
             pp.gt.rw = gt_slot_words(gs.nacc);
             pp.gt.two_words = gs.nparts > 1 ? 1 : 0;
             pp.gt.order_preserving = 0;
-            if (no_join && gs.run_aggregate && key_domain > 0 && key_domain <= ((u64)1 << 34) && !(shuffle && c.world > 1)) {
+            if (no_join && gs.run_aggregate && key_domain > 0 && key_domain <= ((u64)1 << 34) && !(shuffle && c.world > 1) && !op_crowded) {
                 int lg = 0;
                 while (((u64)1 << lg) < cap) lg++;
                 if (lg <= 29) {      // (key - kmin) << log2cap must fit in 64 bits
@@ -1401,7 +1402,10 @@ struct JoinAggPipeline : Pipeline {
             tr.mark("probe+group kernel");
             if (!ovf) break;
             if (attempt > 8) PG_FAIL(PG_ENOMEM, "group table keeps overflowing");
-            cap *= 2;
+            // keys spread unevenly over their domain (a few outliers far from the rest) share a handful of home slots
+            // under the order-preserving map whatever the capacity: hash them instead
+            if (pp.gt.order_preserving) op_crowded = true;
+            else cap *= 2;
         }
         // compact
         const bool do_shuffle = shuffle && c.world > 1;

@@ -53,7 +53,8 @@ vm_scanagg_kernel(const VmAggParams p, i64 *__restrict__ partials /* [grid][G*P]
         if (p.nkeys > 0) g = s_lut[0][p.key0[p.key_side[0] ? row1 : row]];
         if (p.nkeys > 1) g = g * p.n1 + s_lut[1][p.key1[p.key_side[1] ? row1 : row]];
         i64 *t = my + (i64)g * P * NT;
-        if (t[0] == 0) atomicMin((long long *)&s_first[g], (long long)(p.row_base + it));
+        // not "the thread's first row of g": the pre-test queue hands a thread its rows out of order
+        if (p.row_base + it < s_first[g]) atomicMin((long long *)&s_first[g], (long long)(p.row_base + it));
         t[0] += 1;
         for (int a = 0; a < p.nacc; a++) {
             const RvVal v = rv_eval(*p.code, p.a0[a], p.a1[a], row, row1, &err);
