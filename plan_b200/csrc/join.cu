@@ -106,10 +106,13 @@ struct JoinAggPipeline : Pipeline {
     // Group keys functionally dependent on the top join's unique build key (TPC-H Q18 groups by five
     // columns of one orders row): the group table is keyed by the build ROW ID alone and the key columns
     // are fetched once per output group.  kind 0: column of the top build table at that row; kind 1: the
-    // row's `via_key_col` looked up in the rank index of the deeper unique build side `via_stage`.
+    // row's `via_key_col` looked up in the table (rank index or hash table) of the deeper unique build side `via_stage`.
+    // In a star join (`star && fd_mode`) the groups are the rows of lookup `star_anchor - 1` (hits_star_rows_kernel).
     bool fd_mode = false;
     struct FdOut { int kind, slot, col, via_key_col, via_stage; };
     std::vector<FdOut> fd;
+    int fd_stage = -1;                           // the build stage whose row ids the groups are
+    int star_anchor = -1;
     // Star joins (see hits_star_kernel): `main_stage` is the existence join the filter pass tests, `lookups`
     // are all INNER joins of the fact-table spine bottom-up; origin 0 = the fact table, j = lookup j-1's table
     bool star = false;
@@ -169,7 +172,7 @@ struct JoinAggPipeline : Pipeline {
         i64 n = *ngroups, k = topk_limit;
         if (k < 0 || n <= k) return PG_OK;
         if (k == 0) { *ngroups = 0; return PG_OK; }
-        const int planes = gs.nacc + 1;
+        const int planes = gs.nacc + 1 + (int)fd.size();       // dependent keys too: the fast path falls back here after their gather
         constexpr int NB = 1 << TOPK_DIGIT_BITS;
         // hist buffer: [256 bins][min, max as two u64]
         if (!d_hist.p) { PG_TRY(d_hist.alloc(NB * 4 + 16)); PG_TRY(h_hist.alloc(NB * 4 + 16)); }
@@ -1025,6 +1028,43 @@ struct JoinAggPipeline : Pipeline {
         return PG_OK;
     }
 
+    // Sink of a star join grouped by the rows of one lookup: per-row sums in d_dense, compacted into the group list that
+    // finish_groups() takes over (top-k, dependent-key gather, result columns).  A count-only aggregate has no terms: its
+    // sum plane holds zeros that no output reads.
+    int run_star_rows(const StarParams &sp, pg_result *res, Trace &tr)
+    {
+        Context &c = ctx();
+        cudaStream_t st = c.stream;
+        const u64 D = (u64)std::max<i64>(tab(origin_slot[(size_t)star_anchor])->nrows, 1);
+        if (d_dense.bytes < D * 12 + 64) PG_TRY(d_dense.alloc(D * 12 + 64));
+        unsigned long long *dsum = d_dense.as<unsigned long long>();
+        unsigned *dcnt = (unsigned *)(dsum + D);
+        PG_CUDA(cudaMemsetAsync(d_dense.p, 0, D * 12, st));
+        hits_star_rows_kernel<<<c.prop.multiProcessorCount * 8, 256, 0, st>>>(sp, star_anchor, dsum, dcnt);
+        PG_CUDA(cudaGetLastError());
+        PG_CUDA(cudaEventRecord(ev_main.b, st));
+        res->stats.kernel_launches += 2;
+        unsigned long long cnt[4];
+        PG_TRY(read_counters(cnt));
+        tr.mark("star sink (per-row sums)");
+        if (cnt[2] != 0) PG_FAIL(PG_EUNSUPPORTED, "star join: a lookup matched more than one build row (duplicate build keys)");
+        const i64 want = (i64)std::min<u64>(D, std::max<u64>(cnt[1], 1));
+        if (want > out_cap) {
+            PG_TRY(d_out_klo.alloc((size_t)want * 8));
+            PG_TRY(d_out_khi.alloc((size_t)want * 8));
+            PG_TRY(d_out_acc.alloc((size_t)want * 8 * (size_t)(gs.nacc + 1 + (int)fd.size())));    // dependent key columns ride as extra planes
+            out_cap = want;
+        }
+        PG_CUDA(cudaMemsetAsync(d_counters.p, 0, 32, st));
+        dense_compact_kernel<<<(int)std::min<u64>((D + 255) / 256, (u64)c.prop.multiProcessorCount * 8), 256, 0, st>>>(
+            dsum, dcnt, D, 0, d_out_klo.as<i64>(), d_out_khi.as<i64>(), d_out_acc.as<i64>(), out_cap, d_counters.as<unsigned long long>(), -1, 0, 0);
+        PG_CUDA(cudaGetLastError());
+        res->stats.kernel_launches += 1;
+        unsigned long long ng[4];
+        PG_TRY(read_counters(ng));
+        return finish_groups((i64)ng[0], cnt, res, tr);
+    }
+
     // fact-table pipeline of a star join: existence filter pass, then hits_star_kernel (lookups + dense group sums)
     int run_star(pg_result *res, Trace &tr)
     {
@@ -1068,6 +1108,8 @@ struct JoinAggPipeline : Pipeline {
             sp.term[i].mul = sterms[i].mul;
             for (int f = 0; f < sterms[i].nfac; f++) { sp.term[i].fac[f] = href(sterms[i].fac[f]); sp.term[i].fc[f] = sterms[i].fc[f]; sp.term[i].fs[f] = sterms[i].fs[f]; }
         }
+        sp.counters = d_counters.as<unsigned long long>();
+        if (fd_mode) return run_star_rows(sp, res, tr);
         const size_t gbytes = (size_t)star_ngroups * 24;      // sum low word, sum high word, row count
         const int W = (t->dist != PG_DIST_REPLICATED && c.world > 1) ? c.world : 1;
         if (!d_star.p) { PG_TRY(d_star.alloc(gbytes)); PG_TRY(d_star_all.alloc(gbytes * (size_t)c.world)); PG_TRY(h_star.alloc(gbytes * (size_t)c.world)); }
@@ -1075,7 +1117,6 @@ struct JoinAggPipeline : Pipeline {
         sp.gsum = d_star.as<unsigned long long>();
         sp.gsum_hi = sp.gsum + star_ngroups;
         sp.gcnt = sp.gsum + 2 * star_ngroups;
-        sp.counters = d_counters.as<unsigned long long>();
         if ((size_t)star_ngroups * 16 > 48 * 1024)      // above the default dynamic shared memory limit (up to 64 KB at STAR_MAXGROUPS)
             PG_CUDA(cudaFuncSetAttribute(hits_star_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, star_ngroups * 16));
         if (xl >= 0) {
@@ -1429,20 +1470,33 @@ struct JoinAggPipeline : Pipeline {
         ngroups = (i64)ng2[0];
         }
         if (do_shuffle) { PG_TRY(shuffle_groups(&ngroups, pp, res)); tr.mark("all-to-all shuffle + merge"); }
+        return finish_groups(ngroups, cnt, res, tr);
+    }
+
+    // The group list is on the device (d_out_*, ngroups entries, planes [nacc sums][row count][dependent keys]): LIMIT
+    // pre-selection, dependent-key gather, read-back (all-gathered across ranks when the probe side is sharded) and the
+    // result columns.  cnt: the sink's counters {rows passing the filter, joined rows}.
+    int finish_groups(i64 ngroups, const unsigned long long *cnt, pg_result *res, Trace &tr)
+    {
+        Context &c = ctx();
+        cudaStream_t st = c.stream;
+        const pg_table *t = tab(src_slot);
         res->stats.aux[6] = ngroups;          // groups before any LIMIT
         tr.mark("compact");
         if (device_only) { dev_ngroups = ngroups; return PG_OK; }
-        // (FD mode: the ORDER BY keys are fetched below, the host orders the groups)
+        // (FD mode of a plain join has no device top-k: its ORDER BY keys are fetched below and the host orders the groups.
+        // A star join grouped by dimension rows orders by an aggregate: the select runs first and the keys are gathered
+        // for every group, but VARCHARs are only materialised on the host for the candidates that come back.)
         // LIMIT k with a small k over many groups: the radix select runs with its state on the device and the candidates
         // leave in one fixed-size message (below) -- no host round trip per pass
-        const bool topk_fast = has_topk && !fd_mode && topk_limit > 0 && topk_limit <= SG_CAP / 2 && ngroups > topk_limit &&
+        const bool topk_fast = has_topk && topk_limit > 0 && topk_limit <= SG_CAP / 2 && ngroups > topk_limit &&
                                !(getenv("PG_TOPK_HOST") && atoi(getenv("PG_TOPK_HOST")));
-        if (has_topk && !fd_mode && !topk_fast) { PG_TRY(topk_preselect(&ngroups, res)); tr.mark("top-k preselect"); }
+        if (has_topk && !topk_fast) { PG_TRY(topk_preselect(&ngroups, res)); tr.mark("top-k preselect"); }
         if (fd_mode && ngroups > 0) {
             // dependent key columns are written behind the accumulator planes of the group list, so every
             // read-back / cross-rank gather path below carries them like one more aggregate
             const int grid = (int)std::max<i64>(std::min<i64>((ngroups + 255) / 256, (i64)c.prop.multiProcessorCount * 8), 1);
-            const pg_table *bt = tab(stages.back()->src_slot);
+            const pg_table *bt = tab(stages[(size_t)fd_stage]->src_slot);
             for (size_t f = 0; f < fd.size(); f++) {
                 const FdOut &o = fd[f];
                 const pg_table *ct = tab(o.slot);
@@ -1454,7 +1508,7 @@ struct JoinAggPipeline : Pipeline {
                     fd_gather_kernel<<<grid, 256, 0, st>>>(d_out_klo.as<i64>(), ngroups, colref, 0, none, JoinTable{}, none, host_col ? 1 : 0, dst);
                 } else {
                     const Stage &d = *stages[(size_t)o.via_stage];
-                    if (!d.rank_index) PG_FAIL(PG_EUNSUPPORTED, "functionally dependent group key: the deeper build side has no unique-key index");
+                    if (!d.unique_key) PG_FAIL(PG_EUNSUPPORTED, "functionally dependent group key: the deeper build side has no unique key");   // rank index or hash table: one row per key
                     fd_gather_kernel<<<grid, 256, 0, st>>>(d_out_klo.as<i64>(), ngroups, none, 1, typed(bt, o.via_key_col), d.jt, colref,
                                                            host_col ? 1 : 0, dst);
                 }
@@ -1669,6 +1723,7 @@ struct JoinAggPipeline : Pipeline {
                 col.type = cc.type;
                 col.width = cc.width;
                 col.scale = cc.scale;
+                if (cc.type == PG_T_DICT8) col.dict = cc.dict;
                 const int w = type_size(cc.type);
                 col.data.resize((size_t)ngroups * (size_t)w);
                 if (cc.type == PG_T_VARCHAR) {
@@ -2002,23 +2057,24 @@ static int build_star(pg_plan *plan, const Node &aggn, const Node &top, std::uni
     auto mark = [&](const HRef &h) { used[(size_t)h.origin] = true; };
     for (auto &lk : p->lookups) for (int k = 0; k < lk.nkey; k++) mark(lk.key[k]);
 
-    // group keys -> dense index parts
-    if (aggn.groups.empty() || aggn.groups.size() > STAR_MAXPART) PG_FAIL(PG_EUNSUPPORTED, "star join: 1..%d group keys", STAR_MAXPART);
+    // group keys -> dense index parts; keys that do not fit a small dense domain may still name the rows of one dimension
+    std::string dense_why;
     i64 ng = 1;
-    for (auto &g0 : aggn.groups) {
-        const Expr *ge = strip_value_preserving_casts(&g0);
+    if (aggn.groups.empty() || aggn.groups.size() > STAR_MAXPART) dense_why = "1.." + std::to_string(STAR_MAXPART) + " group keys";
+    for (size_t gi = 0; gi < aggn.groups.size() && dense_why.empty(); gi++) {
+        const Expr *ge = strip_value_preserving_casts(&aggn.groups[gi]);
         JoinAggPipeline::HPart hp;
         if (ge->kind == PG_TK_FUNC && ge->fn == PG_FN_EXTRACT && ge->args.size() == 2) {
             const Expr *what = strip_value_preserving_casts(&ge->args[0]), *arg = strip_value_preserving_casts(&ge->args[1]);
-            if (what->kind != PG_TK_STR || what->str != "year") PG_FAIL(PG_EUNSUPPORTED, "only EXTRACT(year ...) is off-loaded");
+            if (what->kind != PG_TK_STR || what->str != "year") { dense_why = "only EXTRACT(year ...) is off-loaded"; break; }
             ge = arg;
             hp.fn = 1;
         }
-        if (ge->kind != PG_TK_COL || !locate(top, ge->idx, &hp.v)) PG_FAIL(PG_EUNSUPPORTED, "star join: group key is not a reachable column");
+        if (ge->kind != PG_TK_COL || !locate(top, ge->idx, &hp.v)) { dense_why = "group key is not a reachable column"; break; }
         const Column &cc = p->tab(p->origin_slot[(size_t)hp.v.origin])->cols[(size_t)hp.v.col];
-        if (cc.any_nulls()) PG_FAIL(PG_EUNSUPPORTED, "star join: nullable group key");
+        if (cc.any_nulls()) { dense_why = "nullable group key"; break; }
         if (hp.fn == 1) {
-            if (cc.type != PG_T_DATE32) PG_FAIL(PG_EUNSUPPORTED, "EXTRACT(year) of a non-date column");
+            if (cc.type != PG_T_DATE32) { dense_why = "EXTRACT(year) of a non-date column"; break; }
             hp.lo = host_year_of_days(cc.gmin());
             hp.n = (int)(host_year_of_days(cc.gmax()) - hp.lo + 1);
             hp.type = PG_T_INT32;
@@ -2031,21 +2087,73 @@ static int build_star(pg_plan *plan, const Node &aggn, const Node &top, std::uni
             hp.n = (int)(cc.gmax() - cc.gmin() + 1);
             hp.type = cc.type;
         } else {
-            PG_FAIL(PG_EUNSUPPORTED, "star join: group key domain is not small and dense");
+            dense_why = "group key domain is not small and dense";
+            break;
         }
         ng *= hp.n;
-        if (ng > STAR_MAXGROUPS) PG_FAIL(PG_EUNSUPPORTED, "star join: more than %d dense groups", STAR_MAXGROUPS);
-        mark(hp.v);
+        if (ng > STAR_MAXGROUPS) { dense_why = "more than " + std::to_string(STAR_MAXGROUPS) + " dense groups"; break; }
         p->sparts.push_back(hp);
     }
-    p->star_ngroups = (int)ng;
+    // Dimension-row groups (TPC-H Q10): every key is a plain column of the build row of one lookup A -- one of them A's unique
+    // build key, the anchor -- or of a lookup B keyed by a column of A's row, with a unique key of its own.  A group is then one
+    // row of A: hits_star_rows_kernel sums per row and the keys are fetched for the groups that come out (as fd_mode does for
+    // plain joins).  Without the anchor, two rows of A could carry equal keys and would have to be merged.
+    auto dimension_rows = [&](std::string *why) -> bool {
+        if (ctx().world > 1) { *why = "runs on one GPU (with a sharded fact table a group's rows span ranks)"; return false; }
+        std::vector<HRef> keys;
+        for (size_t k = 0; k < aggn.groups.size(); k++) {
+            const Expr *ge = strip_value_preserving_casts(&aggn.groups[k]);
+            HRef h;
+            if (ge->kind != PG_TK_COL || !locate(top, ge->idx, &h)) { *why = "group key " + std::to_string(k) + " is not a plain column"; return false; }
+            if (p->tab(p->origin_slot[(size_t)h.origin])->cols[(size_t)h.col].any_nulls()) { *why = "group key " + std::to_string(k) + " is nullable"; return false; }
+            keys.push_back(h);
+        }
+        int a = -1;
+        for (auto &h : keys)
+            if (h.origin > 0 && p->lookups[(size_t)h.origin - 1].nkey == 1 && h.col == p->stages[(size_t)p->lookups[(size_t)h.origin - 1].stage]->ins_key_col) { a = h.origin; break; }
+        if (a < 0) { *why = "no group key is the build key of a joined table (the anchor whose rows would be the groups)"; return false; }
+        const JoinAggPipeline::HLookup &la = p->lookups[(size_t)a - 1];
+        const Stage &A = *p->stages[(size_t)la.stage];
+        const std::string aname = p->tab(A.src_slot)->name;
+        if (!A.unique_key) { *why = "the build key of " + aname + " is not unique"; return false; }
+        std::vector<JoinAggPipeline::FdOut> fd;
+        for (size_t k = 0; k < keys.size(); k++) {
+            const HRef &h = keys[k];
+            if (h.origin == a) { fd.push_back({0, A.src_slot, h.col, -1, -1}); continue; }
+            const JoinAggPipeline::HLookup *lb = h.origin > 0 ? &p->lookups[(size_t)h.origin - 1] : nullptr;
+            if (!lb || lb->key[0].origin != a) { *why = "group key " + std::to_string(k) + " is neither a column of " + aname + " nor of a table joined on one"; return false; }
+            const Stage &B = *p->stages[(size_t)lb->stage];
+            if (lb->nkey != 1) { *why = "group key " + std::to_string(k) + " comes through a two-column join key"; return false; }
+            if (!B.unique_key) { *why = "the build key of " + p->tab(B.src_slot)->name + " is not unique"; return false; }
+            fd.push_back({1, B.src_slot, h.col, lb->key[0].col, lb->stage});
+            used[(size_t)h.origin] = true;
+        }
+        used[(size_t)a] = true;
+        p->fd_mode = true;
+        p->fd = fd;
+        p->fd_stage = la.stage;
+        p->star_anchor = a;
+        p->nparts = p->gs.nparts = 1;
+        return true;
+    };
+    if (dense_why.empty()) {
+        for (auto &hp : p->sparts) mark(hp.v);
+        p->star_ngroups = (int)ng;
+    } else {
+        p->sparts.clear();
+        std::string rows_why;
+        if (!dimension_rows(&rows_why)) PG_FAIL(PG_EUNSUPPORTED, "star join: %s; grouping by dimension rows: %s", dense_why.c_str(), rows_why.c_str());
+    }
 
     // aggregates: one SUM (signed sum of products) and/or COUNT
     p->aggs = aggn.aggs;
     int nsum = 0;
     const AggExpr *sum = nullptr;
     for (auto &ae : aggn.aggs) {
-        if (ae.fn == PG_AGG_COUNT) continue;
+        if (ae.fn == PG_AGG_COUNT) {
+            if (p->fd_mode && ae.ltype != PG_LT_HUGEINT) PG_FAIL(PG_EUNSUPPORTED, "star join: count result type");
+            continue;
+        }
         const bool is_sum = ae.fn == PG_AGG_SUM && (ae.ltype == PG_LT_DECIMAL || ae.ltype == PG_LT_HUGEINT);
         const bool is_avg = ae.fn == PG_AGG_AVG && (ae.ltype == PG_LT_DECIMAL || ae.ltype == PG_LT_DOUBLE);     // sum / row count at result time
         if (!is_sum && !is_avg) PG_FAIL(PG_EUNSUPPORTED, "star join: sum, avg and count only");
@@ -2132,19 +2240,48 @@ static int build_star(pg_plan *plan, const Node &aggn, const Node &top, std::uni
         if ((sum->ltype == PG_LT_HUGEINT || sum->ltype == PG_LT_DOUBLE) && maxs != 0) PG_FAIL(PG_EUNSUPPORTED, "integer sum over a scaled value");
         p->star_scale = maxs;
         p->star_worst = scaled_worst;
-        // a block's shared-memory partial is int64: it receives at most its share of the fact rows (grid-stride over the hits)
-        const i64 threads = (i64)ctx().prop.multiProcessorCount * 8 * 256;
-        const i64 per_block = ((std::max<i64>(st->nrows, 1) + threads - 1) / threads) * 256;
-        if (scaled_worst * (i128)per_block >= ((i128)1 << 63)) PG_FAIL(PG_EUNSUPPORTED, "a block's partial group sum could exceed int64");
+        if (p->fd_mode) {
+            // a dimension row's accumulator is int64 and can receive every fact row
+            if (scaled_worst * (i128)std::max<i64>(st->nrows, 1) >= ((i128)1 << 63)) PG_FAIL(PG_EUNSUPPORTED, "star join grouped by dimension rows: a group sum could exceed int64");
+        } else {
+            // a block's shared-memory partial is int64: it receives at most its share of the fact rows (grid-stride over the hits)
+            const i64 threads = (i64)ctx().prop.multiProcessorCount * 8 * 256;
+            const i64 per_block = ((std::max<i64>(st->nrows, 1) + threads - 1) / threads) * 256;
+            if (scaled_worst * (i128)per_block >= ((i128)1 << 63)) PG_FAIL(PG_EUNSUPPORTED, "a block's partial group sum could exceed int64");
+        }
+    }
+    if (p->fd_mode) {
+        if (st->nrows >= ((i64)1 << 32)) PG_FAIL(PG_EUNSUPPORTED, "star join grouped by dimension rows: 2^32 fact rows or more (the per-row count is 32-bit)");
+        // the group list of finish_groups(): one sum plane (zeros for a count-only aggregate), then the row-count plane
+        p->gs.nacc = 1;
+        p->agg_plane.assign(aggn.aggs.size(), 1);
+        p->agg_scale.assign(aggn.aggs.size(), 0);
+        for (size_t i = 0; i < aggn.aggs.size(); i++)
+            if (aggn.aggs[i].fn != PG_AGG_COUNT) { p->agg_plane[i] = 0; p->agg_scale[i] = p->star_scale; }
     }
     for (size_t o = 1; o < used.size(); o++) p->stages[(size_t)p->lookups[o - 1].stage]->payload_needed = used[o];
     for (auto &o : aggn.outs) {
-        if (o.first == 0 && (o.second < 0 || o.second >= (int)p->sparts.size())) PG_FAIL(PG_EUNSUPPORTED, "bad group output index");
+        if (o.first == 0 && (o.second < 0 || o.second >= (int)(p->fd_mode ? p->fd.size() : p->sparts.size()))) PG_FAIL(PG_EUNSUPPORTED, "bad group output index");
         if (o.first == 1 && (o.second < 0 || o.second >= (int)aggn.aggs.size())) PG_FAIL(PG_EUNSUPPORTED, "bad aggregate output index");
         if (o.first != 0 && o.first != 1) PG_FAIL(PG_EUNSUPPORTED, "bad output kind");
     }
     p->outs = aggn.outs;
     if (aggn.having.size()) PG_FAIL(PG_EUNSUPPORTED, "star join: HAVING");
+    if (p->fd_mode && plan->topk && !plan->topk->order.empty()) {
+        // ORDER BY an aggregate ... LIMIT k: device pre-selection on the sum plane, so that only the candidates' keys reach the host
+        const auto o = aggn.outs[(size_t)plan->topk->order[0].first];
+        if (o.first == 1 && aggn.aggs[(size_t)o.second].fn != PG_AGG_AVG) {
+            TopkKey tk{};
+            tk.desc = plan->topk->order[0].second ? 1 : 0;
+            tk.div = 1;
+            tk.src = 3;
+            tk.plane = p->agg_plane[(size_t)o.second];
+            for (int i = 2; i < p->agg_scale[(size_t)o.second]; i++) tk.div *= 10;     // DECIMAL keys compare at two fractional digits
+            p->has_topk = true;
+            p->topk_key = tk;
+            p->topk_limit = plan->topk->limit;
+        }
+    }
     // bytes: the filter pass streams the fact key (+ predicate) column; everything else is gathered per hit
     p->main_bytes = st->nrows * st->cols[(size_t)p->probe_key_col].phys_width();
     for (auto &r : p->ranges) p->main_bytes += st->nrows * st->cols[(size_t)r.col].phys_width();
@@ -2222,7 +2359,7 @@ static int build_star(pg_plan *plan, const Node &aggn, const Node &top, std::uni
     if (must_x.size() == 1) {
         if (!x_candidate(must_x[0])) PG_FAIL(PG_EUNSUPPORTED, "sharded join sides are not co-partitioned on the key and the row exchange does not apply: %s", x_why.c_str());
         p->xl = (int)must_x[0];
-    } else if (force_x) {
+    } else if (force_x && !p->fd_mode) {        // per-row groups are summed where the hit is: never exchanged
         // prefer a join whose build columns the aggregate reads (there is something to carry)
         for (int pass = 0; pass < 2 && p->xl < 0; pass++)
             for (size_t l : may_x)
@@ -2247,7 +2384,8 @@ static int build_star(pg_plan *plan, const Node &aggn, const Node &top, std::uni
     }
     PG_TRY(p->d_counters.alloc(128));
     PG_TRY(p->d_overflow.alloc(4));
-    std::string ex = "StarJoin[existence filter -> per-hit lookups -> dense shared-memory groups] kernel=filter_hits_kernel+hits_star_kernel fact=" + st->name + " joins:";
+    std::string ex = p->fd_mode ? "StarJoin[existence filter -> per-hit lookups -> per-row global sums] kernel=filter_hits_kernel+hits_star_rows_kernel fact=" + st->name + " joins:"
+                                : "StarJoin[existence filter -> per-hit lookups -> dense shared-memory groups] kernel=filter_hits_kernel+hits_star_kernel fact=" + st->name + " joins:";
     for (size_t l = 0; l < p->lookups.size(); l++) {
         const Stage &S = *p->stages[(size_t)p->lookups[l].stage];
         char b[200];
@@ -2255,8 +2393,12 @@ static int build_star(pg_plan *plan, const Node &aggn, const Node &top, std::uni
                  S.payload_needed ? ", payload" : ", existence", (int)l == p->xl ? ", ROW EXCHANGE: both sides hash-partitioned on the key, all-to-all over NVLink, joined on the owner rank" : "");
         ex += b;
     }
-    char b[96];
-    snprintf(b, sizeof b, " groups=%d (dense) terms=%zu", p->star_ngroups, p->sterms.size());
+    char b[160];
+    if (p->fd_mode)
+        snprintf(b, sizeof b, " groups=rows of %s (dependent keys fetched per group) terms=%zu%s", p->tab(p->origin_slot[(size_t)p->star_anchor])->name.c_str(),
+                 p->sterms.size(), p->has_topk ? " top-k=device" : "");
+    else
+        snprintf(b, sizeof b, " groups=%d (dense) terms=%zu", p->star_ngroups, p->sterms.size());
     p->explain = ex + b;
     *out = std::move(p);
     return PG_OK;
@@ -2405,6 +2547,7 @@ int build_join_agg(pg_plan *plan, const Node &aggn, const Node &top, std::unique
         if (ok && anchor && need) {
             p->fd_mode = true;
             p->fd = fd;
+            p->fd_stage = top_stage;
             for (auto &f : fd) if (f.kind == 1) p->stages[(size_t)f.via_stage]->payload_needed = true;
         }
     }

@@ -1146,6 +1146,47 @@ __device__ __forceinline__ i64 year_of_days(i64 z)
     return y + (mp >= 10 ? 1 : 0);
 }
 
+// The joins of hit i: rows[0] = its fact row, rows[l + 1] = the build row lookup l matched (-1 for an existence lookup).
+// False when some join finds no build row; a lookup with more than one match counts into n_multi.
+__device__ __forceinline__ bool star_lookups(const StarParams &sp, unsigned long long i, i64 (&rows)[STAR_MAXLOOKUP + 1], unsigned long long &n_multi)
+{
+    rows[0] = (i64)sp.hits[i];
+    auto val = [&](const ValRef &r) { return load_typed(r.col, rows[r.from_build]); };
+    bool ok = true;
+#pragma unroll
+    for (int l = 0; l < STAR_MAXLOOKUP; l++) {
+        if (l >= sp.nlookup || !ok) continue;
+        const StarLookup &L = sp.lk[l];
+        i64 key = val(L.key[0]);
+        if (L.nkey == 2) key = (key << 32) | (val(L.key[1]) & 0xffffffffLL);
+        rows[l + 1] = -1;
+        if (L.existence) {
+            ok = bitmap_test(L.jt, key);
+        } else {
+            int matches = 0;
+            jt_probe(L.jt, key, [&](u64 r) { rows[l + 1] = (i64)r; matches++; });
+            ok = matches > 0;
+            n_multi += matches > 1 ? 1 : 0;
+        }
+    }
+    return ok;
+}
+
+// the summed value of one joined row: sum over the terms of mul * prod(fc + fs * value)
+__device__ __forceinline__ i64 star_amount(const StarParams &sp, const i64 (&rows)[STAR_MAXLOOKUP + 1])
+{
+    auto val = [&](const ValRef &r) { return load_typed(r.col, rows[r.from_build]); };
+    i64 amount = 0;
+#pragma unroll
+    for (int t = 0; t < STAR_MAXTERM; t++) {
+        if (t >= sp.nterm) continue;
+        i64 x = sp.term[t].mul;
+        for (int f = 0; f < sp.term[t].nfac; f++) x *= sp.term[t].fc[f] + sp.term[t].fs[f] * val(sp.term[t].fac[f]);
+        amount += x;
+    }
+    return amount;
+}
+
 static __global__ void __launch_bounds__(256)
 hits_star_kernel(const StarParams sp)
 {
@@ -1157,27 +1198,9 @@ hits_star_kernel(const StarParams sp)
     unsigned long long n_join = 0, n_multi = 0;
     for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
         i64 rows[STAR_MAXLOOKUP + 1];
-        rows[0] = (i64)sp.hits[i];
-        auto val = [&](const ValRef &r) { return load_typed(r.col, rows[r.from_build]); };
-        bool ok = true;
-#pragma unroll
-        for (int l = 0; l < STAR_MAXLOOKUP; l++) {
-            if (l >= sp.nlookup || !ok) continue;
-            const StarLookup &L = sp.lk[l];
-            i64 key = val(L.key[0]);
-            if (L.nkey == 2) key = (key << 32) | (val(L.key[1]) & 0xffffffffLL);
-            rows[l + 1] = -1;
-            if (L.existence) {
-                ok = bitmap_test(L.jt, key);
-            } else {
-                int matches = 0;
-                jt_probe(L.jt, key, [&](u64 r) { rows[l + 1] = (i64)r; matches++; });
-                ok = matches > 0;
-                n_multi += matches > 1 ? 1 : 0;
-            }
-        }
-        if (!ok) continue;
+        if (!star_lookups(sp, i, rows, n_multi)) continue;
         n_join++;
+        auto val = [&](const ValRef &r) { return load_typed(r.col, rows[r.from_build]); };
         int g = 0;
 #pragma unroll
         for (int k = 0; k < STAR_MAXPART; k++) {
@@ -1186,14 +1209,7 @@ hits_star_kernel(const StarParams sp)
             if (sp.part[k].fn == 1) v = year_of_days(v);
             g = g * sp.part[k].n + (int)(v - sp.part[k].lo);
         }
-        i64 amount = 0;
-#pragma unroll
-        for (int t = 0; t < STAR_MAXTERM; t++) {
-            if (t >= sp.nterm) continue;
-            i64 x = sp.term[t].mul;
-            for (int f = 0; f < sp.term[t].nfac; f++) x *= sp.term[t].fc[f] + sp.term[t].fs[f] * val(sp.term[t].fac[f]);
-            amount += x;
-        }
+        const i64 amount = star_amount(sp, rows);
         atomicAdd(&s_sum[g], (unsigned long long)amount);
         atomicAdd(&s_cnt[g], 1ULL);
     }
@@ -1207,6 +1223,32 @@ hits_star_kernel(const StarParams sp)
             if (hi) atomicAdd(&sp.gsum_hi[i], (unsigned long long)hi);
             atomicAdd(&sp.gcnt[i], s_cnt[i]);
         }
+    }
+    n_join = (unsigned long long)warp_sum((i64)n_join);
+    n_multi = (unsigned long long)warp_sum((i64)n_multi);
+    if ((threadIdx.x & 31) == 0) {
+        if (n_join) atomicAdd(&sp.counters[1], n_join);
+        if (n_multi) atomicAdd(&sp.counters[2], n_multi);
+    }
+}
+
+// Star join grouped by the build ROW of one lookup (TPC-H Q10: the customer row; every group key is a column of that row or
+// of a unique lookup keyed from it).  Same joins and amount as hits_star_kernel, but the groups are as many as that table's
+// rows: the sink adds into global per-row accumulators dsum[row] (u64, the host proved the total fits int64) and
+// dcnt[row] (u32, fewer than 2^32 fact rows) -- the layout of group1_dense_kernel, compacted by dense_compact_kernel.
+// `anchor` indexes rows[]: 1 + the lookup whose row is the group.
+static __global__ void __launch_bounds__(256)
+hits_star_rows_kernel(const StarParams sp, int anchor, unsigned long long *__restrict__ dsum, unsigned *__restrict__ dcnt)
+{
+    const unsigned long long n = *sp.hit_count;
+    unsigned long long n_join = 0, n_multi = 0;
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
+        i64 rows[STAR_MAXLOOKUP + 1];
+        if (!star_lookups(sp, i, rows, n_multi)) continue;
+        n_join++;
+        const u64 g = (u64)rows[anchor];
+        atomicAdd(dsum + g, (unsigned long long)star_amount(sp, rows));
+        atomicAdd(dcnt + g, 1u);
     }
     n_join = (unsigned long long)warp_sum((i64)n_join);
     n_multi = (unsigned long long)warp_sum((i64)n_multi);

@@ -761,10 +761,12 @@ Q10_CUSTOMER = [("c_custkey", L.PG_T_INT32, 0, 0, None), ("c_name", L.PG_T_VARCH
                 ("c_comment", L.PG_T_VARCHAR, 117, 0, None)]
 
 
-def q10_plan(date_lo=None, date_hi=None, limit=20):
+def q10_plan(date_lo=None, date_hi=None, limit=20, agg="sum"):
     """cases/tpch/query/q10.sql:  Limit(20) <- Order(revenue desc) <- Agg(group by c_custkey, c_name, c_acctbal, c_phone, n_name,
     c_address, c_comment; sum(l_extendedprice * (1 - l_discount))) <- lineitem[l_returnflag = 'R'] x orders[o_orderdate in the
-    quarter] x customer x nation.  Seven group keys, four of them strings, one a signed DECIMAL.  Plan tree only (see Q5 / Q7 / Q8)."""
+    quarter] x customer x nation.  Seven group keys, four of them strings, one a signed DECIMAL.  The GPU runs it as a star join
+    grouped by customer rows (every key depends on the customer row; n_name through c_nationkey), with the ORDER BY ... LIMIT
+    pre-selected on the device.  limit=None: the bare aggregate.  agg="avg": avg(DECIMAL) = sum.Quo(count), plus count(*)."""
     B, V, D = K.LType(K.LTID_BOOLEAN), K.VarcharType(), K.DateType()
     date_lo = days(1993, 3, 1) if date_lo is None else date_lo
     date_hi = days(1993, 6, 1) if date_hi is None else date_hi
@@ -777,9 +779,14 @@ def q10_plan(date_lo=None, date_hi=None, limit=20):
     st.join("nation", [("c_nationkey", "n_nationkey")], ["n_name"])
     keys = [st.ref(n) for n in ("c_custkey", "c_name", "c_acctbal", "c_phone", "n_name", "c_address", "c_comment")]
     sum_t = K.DecimalType(38, 4)
-    agg = func("sum", sum_t, _disc_price(st.ref("l_extendedprice"), st.ref("l_discount")))
+    aggs = [func(agg, sum_t, _disc_price(st.ref("l_extendedprice"), st.ref("l_discount")))]
     # select list order: c_custkey, c_name, revenue, c_acctbal, n_name, c_address, c_phone, c_comment
     outs = [col(0, 0, keys[0].DataTyp), col(0, 1, V), col(1, 0, sum_t), col(0, 2, keys[2].DataTyp), col(0, 4, V), col(0, 5, V), col(0, 3, V), col(0, 6, V)]
-    node = PhysicalOperator(POT_Agg, Outputs=outs, Children=[st.node], Info=AggOpInfo([agg], keys))
+    if agg == "avg":
+        aggs.append(func("count", K.HugeintType(), st.ref("l_orderkey")))
+        outs.append(col(1, 1, K.HugeintType()))
+    node = PhysicalOperator(POT_Agg, Outputs=outs, Children=[st.node], Info=AggOpInfo(aggs, keys))
+    if limit is None:
+        return node
     order = PhysicalOperator(POT_Order, Outputs=outs, Children=[node], Info=OrderOpInfo([(col(0, 2, sum_t), True)]))
     return PhysicalOperator(POT_Limit, Outputs=outs, Children=[order], Info=LimitOpInfo(limit))
