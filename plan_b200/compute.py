@@ -232,12 +232,27 @@ class DeviceTable:
         return cls(name, h, columns)
 
     def append(self, arrays, valid=None):
-        """arrays: one contiguous numpy array (or raw pointer int) per column, host memory."""
+        """arrays: one contiguous numpy array (or raw pointer int) per column, host memory.  A VARCHAR column is a list / array of
+        bytes or str, or a (blob uint8 array, offsets int64 array of n + 1) pair: row r is blob[offsets[r]:offsets[r + 1]]."""
         lib = L.lib()
         n = len(self.columns)
         ptrs = (C.c_void_p * n)()
         nrows = None
         for i, a in enumerate(arrays):
+            if self.columns[i][1] == L.PG_T_VARCHAR and isinstance(a, tuple) and len(a) == 2 and all(isinstance(x, np.ndarray) for x in a):
+                blob, off = np.ascontiguousarray(a[0], dtype=np.uint8), np.asarray(a[1], dtype=np.int64)
+                if off.ndim != 1 or len(off) < 1 or (len(off) > 1 and (off[0] < 0 or off[-1] > len(blob) or (np.diff(off) < 0).any())):
+                    raise ValueError("VARCHAR column %s: offsets must be n + 1 non-decreasing positions inside the blob" % self.columns[i][0])
+                if len(blob) == 0:
+                    blob = np.zeros(1, np.uint8)          # a valid address for empty strings
+                sv = np.empty(len(off) - 1, dtype=K.PG_STRING)
+                sv["len"] = np.diff(off)
+                sv["data"] = blob.ctypes.data + off[:-1].astype(np.uint64)
+                arrays[i] = (sv, blob)
+                ptrs[i] = sv.ctypes.data
+                nrows = len(sv) if nrows is None else nrows
+                assert len(sv) == nrows
+                continue
             if self.columns[i][1] == L.PG_T_VARCHAR:
                 # list / array of bytes|str -> one pg_string per row over a single contiguous buffer
                 raw = [x.encode() if isinstance(x, str) else bytes(x) for x in a]

@@ -18,6 +18,7 @@
 #include "hostdec.hpp"
 #include "join.cuh"
 #include "exchange.cuh"
+#include "leftcount.cuh"
 #include "pipeline.hpp"
 
 namespace pg {
@@ -2862,6 +2863,348 @@ no_device_topk:
                  p->shuffle ? " exchange=all-to-all(hash-partitioned)" : "");
     if (p->no_join) ex = b; else ex += b;
     p->explain = ex;
+    *out = std::move(p);
+    return PG_OK;
+}
+
+}  // namespace pg
+
+// ------------------------------------------------------------------ grouped LEFT-join count (leftcount.cuh) --
+//
+// `Agg(group by k; count(x)) <- LeftJoin(k = fk) <- {Scan(preserved), Scan(build)}`, alone or under
+// `Agg(group by that count; count(*))` (TPC-H Q13).  A group is one row of the preserved side that passes its filters; its
+// key k is the anchor.  The preserved side becomes a key table (the ordinary build stage: rank index, identity rank index
+// or hash table; payload = row id), the build side is streamed once into a u32 count per preserved row.
+// count(build column) is the number of matched rows whose argument is non-NULL, NULL when that is 0 (CountOp.Finalize over
+// the NULL-padded row); count(*) and count(non-null preserved column) are max(matches, 1).
+
+namespace pg {
+
+namespace {
+
+struct LeftCountPipeline : Pipeline {
+    JoinAggPipeline jp;                  // plan, tables and stage 0: the preserved side's key table and its build machinery
+    int anchor_col = -1;                 // the preserved side's join key
+    int build_slot = -1, build_key_col = -1;
+    int arg_col = -1;                    // count(build column): its column; -1: every matched row counts
+    bool null_if_empty = false;          // count(build column): 0 matches is NULL, otherwise max(matches, 1)
+    bool outer = false;                  // Agg(group by count; count(*)) on top
+    std::vector<Range> build_ranges;
+    std::vector<std::pair<int, int>> outs;
+    LcFilter fa{}, fb{};                 // preserved-side (group) and build-side filters
+    DevBuf d_counts, d_cnt, d_hist, d_out_key, d_out_cnt;
+    i64 big_cap = 0;
+    EventPair ev_all, ev_main;
+    i64 main_bytes = 0, algorithmic_bytes = 0;
+
+    // range / code-set predicates and string predicates of one scan; desc: what each string predicate runs as
+    int fill(LcFilter &f, const std::vector<Range> &rs, int slot, std::vector<std::string> *desc)
+    {
+        const pg_table *t = jp.tab(slot);
+        const bool bytewise = getenv("PG_LIKE_BYTEWISE") && atoi(getenv("PG_LIKE_BYTEWISE")) != 0;
+        f.npred = f.nlike = 0;
+        for (auto &r : rs) {
+            if (!r.like) {
+                if (f.npred >= PIPE_MAXPRED) PG_FAIL(PG_EUNSUPPORTED, "more than %d predicate columns on one scan", PIPE_MAXPRED);
+                SrcPred &q = f.pred[f.npred++];
+                q.col = typed(t, r.col);
+                q.lo = r.lo;
+                q.hi = r.hi;
+                q.is_set = r.is_set ? 1 : 0;
+                memcpy(q.mask, r.set, sizeof q.mask);
+                continue;
+            }
+            const Column &col = t->cols[(size_t)r.col];
+            if (!col.d_off) PG_FAIL(PG_EUNSUPPORTED, "string predicate on %s without a device copy of the text", col.name.c_str());
+            if (f.nlike >= GEN_MAXLIKE) PG_FAIL(PG_EUNSUPPORTED, "more than %d string predicates on one scan", GEN_MAXLIKE);
+            GenLike &l = f.like[f.nlike++];
+            memset(&l, 0, sizeof l);
+            l.bytes = col.d_bytes;
+            l.off = (const i64 *)col.d_off;
+            std::vector<std::string> segs;
+            if (r.like <= 2 && !bytewise && like_segments(r.pat, &segs)) {
+                l.kind = r.like == 1 ? GEN_LIKE_WORDS : GEN_NOTLIKE_WORDS;
+                l.plen = (int)segs.size();
+                for (size_t s = 0; s < segs.size(); s++) {
+                    memcpy(l.pat + 8 * s, segs[s].data(), segs[s].size());
+                    l.pat[32 + s] = (char)segs[s].size();
+                }
+                if (desc) desc->push_back(std::to_string(segs.size()) + "-segment word search");
+                continue;
+            }
+            if (r.pat.size() > GEN_PATMAX) PG_FAIL(PG_EUNSUPPORTED, "string pattern longer than %d bytes", GEN_PATMAX);
+            l.kind = r.like;
+            l.plen = (int)r.pat.size();
+            memcpy(l.pat, r.pat.data(), r.pat.size());
+            if (desc) desc->push_back(r.like <= 2 ? "byte-wise wildcard match" : "byte equality");
+        }
+        return PG_OK;
+    }
+
+    int run(pg_result *res) override
+    {
+        Context &c = ctx();
+        cudaStream_t st = c.stream;
+        PG_TRY(ev_all.init());
+        PG_TRY(ev_main.init());
+        Trace tr("leftcount");
+        PG_CUDA(cudaEventRecord(ev_all.a, st));
+        res->stats.kernel_launches = 0;
+        jp.cur_res = res;
+        jp.deferred_stats = 0;
+        PG_CUDA(cudaMemsetAsync(jp.d_counters.p, 0, 128, st));
+        Stage &A = *jp.stages[0];
+        PG_TRY(jp.run_build_stage(A, res, 0));
+        tr.mark("build stage (preserved keys)");
+        const pg_table *at = jp.tab(A.src_slot), *bt = jp.tab(build_slot);
+        if (!A.unique_key && !A.rank_index) {
+            // the statistics do not prove the preserved keys unique: every built row must find itself and nothing else
+            PipeParams pp{};
+            pp.nrows = at->nrows;
+            PG_TRY(jp.fill_preds(pp, A.ranges, A.src_slot));
+            pp.has_probe = 1;
+            pp.probe_key = typed(at, anchor_col);
+            pp.probe = A.jt;
+            pp.counters = jp.d_counters.as<unsigned long long>();
+            PG_CUDA(cudaMemsetAsync(jp.d_counters.p, 0, 32, st));
+            PG_TRY(jp.launch_pipe<SINK_COUNT>(pp, at));
+            res->stats.kernel_launches += 1;
+            unsigned long long k[4];
+            PG_TRY(jp.read_counters(k));
+            if (k[1] != k[0]) PG_FAIL(PG_EUNSUPPORTED, "left-join count: the preserved side holds a key more than once (duplicate %s.%s)",
+                                      at->name.c_str(), at->cols[(size_t)anchor_col].name.c_str());
+            tr.mark("preserved keys unique");
+        }
+        const i64 D = std::max<i64>(at->nrows, 1);
+        if (d_counts.bytes < (size_t)D * 4) PG_TRY(d_counts.alloc((size_t)D * 4));
+        if (!d_cnt.p) PG_TRY(d_cnt.alloc(32));
+        PG_CUDA(cudaMemsetAsync(d_counts.p, 0, (size_t)D * 4, st));
+        PG_CUDA(cudaMemsetAsync(d_cnt.p, 0, 32, st));
+        LeftCountParams p{};
+        p.nrows = bt->nrows;
+        p.f = fb;
+        p.key = typed(bt, build_key_col);
+        if (arg_col >= 0) p.arg = typed(bt, arg_col);
+        p.anchor = A.jt;
+        p.counts = d_counts.as<unsigned>();
+        p.counters = d_cnt.as<unsigned long long>();
+        unsigned long long *cnt = d_cnt.as<unsigned long long>();
+        const int grid = c.prop.multiProcessorCount * 8;
+        PG_CUDA(cudaEventRecord(ev_main.a, st));
+        left_count_kernel<<<grid, 256, 0, st>>>(p);
+        PG_CUDA(cudaGetLastError());
+        PG_CUDA(cudaEventRecord(ev_main.b, st));
+        res->stats.kernel_launches += 1;
+        tr.mark("left_count_kernel");
+        unsigned long long h_cnt[4];
+        auto count_value = [&](u64 m) { return null_if_empty ? m : std::max<u64>(m, 1); };    // 0 = NULL (count(build column) only)
+        ResCol kcol, ccol;
+        if (outer) {
+            const size_t words = (size_t)LC_HBINS + 1 + (size_t)big_cap;
+            if (d_hist.bytes < words * 4) PG_TRY(d_hist.alloc(words * 4));
+            unsigned *hist = d_hist.as<unsigned>();
+            PG_CUDA(cudaMemsetAsync(hist, 0, ((size_t)LC_HBINS + 1) * 4, st));
+            count_hist_kernel<<<JoinAggPipeline::grid_rows(at->nrows), 256, 0, st>>>(fa, at->nrows, d_counts.as<unsigned>(), hist, hist + LC_HBINS,
+                                                                                     hist + LC_HBINS + 1, (unsigned)big_cap);
+            PG_CUDA(cudaGetLastError());
+            res->stats.kernel_launches += 1;
+            std::vector<unsigned> h((size_t)LC_HBINS + 1);
+            PG_CUDA(cudaMemcpyAsync(h.data(), hist, h.size() * 4, cudaMemcpyDeviceToHost, st));
+            PG_CUDA(cudaMemcpyAsync(h_cnt, cnt, 32, cudaMemcpyDeviceToHost, st));
+            PG_CUDA(cudaEventRecord(ev_all.b, st));
+            PG_CUDA(cudaStreamSynchronize(st));
+            const u64 nbig = h[LC_HBINS];
+            if (nbig > (u64)big_cap) PG_FAIL(PG_ECUDA, "internal: more large counts than counted rows allow");
+            std::vector<unsigned> big((size_t)nbig);
+            if (nbig) {
+                PG_CUDA(cudaMemcpyAsync(big.data(), hist + LC_HBINS + 1, (size_t)nbig * 4, cudaMemcpyDeviceToHost, st));
+                PG_CUDA(cudaStreamSynchronize(st));
+                std::sort(big.begin(), big.end());
+            }
+            tr.mark("count_hist_kernel + d2h");
+            // (c_count, custdist): the distinct values of the inner count and how many groups have each
+            std::vector<std::pair<u64, u64>> dist;
+            auto add = [&](u64 v, u64 n) {
+                if (!n) return;
+                if (!dist.empty() && dist.back().first == v) dist.back().second += n;
+                else dist.push_back({v, n});
+            };
+            for (int b = 0; b < LC_HBINS; b++) add(count_value((u64)b), h[(size_t)b]);
+            for (unsigned v : big) add(v, 1);
+            res->nrows = (i64)dist.size();
+            kcol.type = ccol.type = PG_T_HUGEINT;
+            for (auto &d : dist) {
+                const size_t i = kcol.data.size() / sizeof(pg_hugeint);
+                if (d.first == 0) kcol.push_null(i, sizeof(pg_hugeint));
+                else { kcol.push(pg_hugeint{d.first, 0}); kcol.mark_valid(); }
+                ccol.push(pg_hugeint{d.second, 0});
+            }
+        } else {
+            if (d_out_key.bytes < (size_t)D * 8) { PG_TRY(d_out_key.alloc((size_t)D * 8)); PG_TRY(d_out_cnt.alloc((size_t)D * 4)); }
+            left_compact_kernel<<<JoinAggPipeline::grid_rows(at->nrows), 256, 0, st>>>(fa, at->nrows, typed(at, anchor_col), d_counts.as<unsigned>(),
+                                                                                       d_out_key.as<i64>(), d_out_cnt.as<unsigned>(), cnt + 2);
+            PG_CUDA(cudaGetLastError());
+            res->stats.kernel_launches += 1;
+            PG_CUDA(cudaMemcpyAsync(h_cnt, cnt, 32, cudaMemcpyDeviceToHost, st));
+            PG_CUDA(cudaStreamSynchronize(st));
+            const i64 n = (i64)h_cnt[2];
+            std::vector<i64> keys((size_t)n);
+            std::vector<unsigned> counts((size_t)n);
+            if (n) {
+                PG_CUDA(cudaMemcpyAsync(keys.data(), d_out_key.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+                PG_CUDA(cudaMemcpyAsync(counts.data(), d_out_cnt.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+            }
+            PG_CUDA(cudaEventRecord(ev_all.b, st));
+            PG_CUDA(cudaStreamSynchronize(st));
+            tr.mark("left_compact_kernel + d2h");
+            res->nrows = n;
+            kcol.type = at->cols[(size_t)anchor_col].type;
+            const size_t w = (size_t)type_size(kcol.type);
+            kcol.data.resize((size_t)n * w);
+            ccol.type = PG_T_HUGEINT;
+            ccol.data.resize((size_t)n * sizeof(pg_hugeint));
+            pg_hugeint *cv = (pg_hugeint *)ccol.data.data();
+            for (i64 i = 0; i < n; i++) {
+                if (w == 4) ((int32_t *)kcol.data.data())[i] = (int32_t)keys[(size_t)i];
+                else ((i64 *)kcol.data.data())[i] = keys[(size_t)i];
+                const u64 v = count_value(counts[(size_t)i]);
+                cv[i].lower = v;
+                cv[i].upper = 0;
+                if (v == 0) {
+                    if (ccol.valid.empty()) ccol.valid.assign((size_t)n, 1);
+                    ccol.valid[(size_t)i] = 0;
+                }
+            }
+        }
+        for (auto &o : outs) res->cols.push_back(o.first == 0 ? kcol : ccol);
+        res->stats.aux[0] = (i64)h_cnt[0];
+        res->stats.aux[1] = (i64)h_cnt[1];
+        res->stats.aux[6] = res->nrows;
+        res->stats.rows_scanned = bt->nrows;
+        res->stats.kernel_ms = ev_all.ms();
+        res->stats.main_kernel_ms = ev_main.ms();
+        res->stats.algorithmic_bytes = algorithmic_bytes;
+        res->stats.main_kernel_bytes = main_bytes;
+        tr.mark("result columns");
+        return PG_OK;
+    }
+};
+
+}  // namespace
+
+// Agg(k; count) <- LeftJoin, optionally under Agg(count; count(*)): `root` is the topmost aggregate.  Tried only where the
+// other join-aggregate pipelines refuse; every refusal is PG_EUNSUPPORTED with its reason.
+int build_left_count(pg_plan *plan, const Node &root, std::unique_ptr<Pipeline> *out)
+{
+    std::unique_ptr<LeftCountPipeline> p(new LeftCountPipeline());
+    p->jp.plan = plan;
+    const Node *inner = &root, *x = &root.children[0];
+    bool filtered = false;
+    while (x->op == PG_OP_FILTER) { filtered = true; x = &x->children[0]; }
+    if (x->op == PG_OP_AGG) {
+        if (filtered) PG_FAIL(PG_EUNSUPPORTED, "a filter between the two aggregates (HAVING on the inner one)");
+        p->outer = true;
+        inner = x;
+        x = &inner->children[0];
+        while (x->op == PG_OP_FILTER) { filtered = true; x = &x->children[0]; }
+        if (root.having.size()) PG_FAIL(PG_EUNSUPPORTED, "HAVING on the outer aggregate");
+    }
+    if (inner->having.size()) PG_FAIL(PG_EUNSUPPORTED, "HAVING on the per-group count");
+    if (x->op != PG_OP_JOIN) PG_FAIL(PG_EUNSUPPORTED, p->outer ? "an aggregate over an aggregate whose input is not a join" : "the aggregate's input is not a join");
+    if (filtered) PG_FAIL(PG_EUNSUPPORTED, "a filter between the aggregate and the join");
+    const Node &J = *x;
+    if (J.jointype != PG_JOIN_LEFT) PG_FAIL(PG_EUNSUPPORTED, "the join is not a LEFT join");
+    if (J.conds.size() != 1) PG_FAIL(PG_EUNSUPPORTED, "the join key has more than one column");
+    if (ctx().world > 1) PG_FAIL(PG_EUNSUPPORTED, "runs on one GPU (a preserved row's matches span ranks; per-rank counts are not merged)");
+    const Node *ps = &J.children[0], *bs = &J.children[1];
+    std::vector<Expr> bf;
+    while (ps->op == PG_OP_FILTER) ps = &ps->children[0];
+    while (bs->op == PG_OP_FILTER) { for (auto &f : bs->filters) bf.push_back(f); bs = &bs->children[0]; }
+    if (ps->op != PG_OP_SCAN) PG_FAIL(PG_EUNSUPPORTED, "the preserved side is not a scan");
+    if (bs->op != PG_OP_SCAN) PG_FAIL(PG_EUNSUPPORTED, "the build side is not a scan");
+    const Expr *pe = strip_value_preserving_casts(&J.conds[0].first), *be = strip_value_preserving_casts(&J.conds[0].second);
+    BaseCol pk, bk;
+    if (pe->kind != PG_TK_COL || be->kind != PG_TK_COL || !resolve(J.children[0], pe->idx, &pk) || !resolve(J.children[1], be->idx, &bk) ||
+        pk.slot != ps->slot || bk.slot != bs->slot)
+        PG_FAIL(PG_EUNSUPPORTED, "join condition is not column = column");
+    const pg_table *at = p->jp.tab(pk.slot), *bt = p->jp.tab(bk.slot);
+    const Column &ac = at->cols[(size_t)pk.col];
+    if (ac.type != PG_T_INT32 && ac.type != PG_T_INT64) PG_FAIL(PG_EUNSUPPORTED, "the anchor key %s is not an integer column", ac.name.c_str());
+    if (ac.any_nulls()) PG_FAIL(PG_EUNSUPPORTED, "the anchor key %s is nullable", ac.name.c_str());
+    if (!is_int_family(bt->cols[(size_t)bk.col].type)) PG_FAIL(PG_EUNSUPPORTED, "the build side's join key is not an integer column");
+    // the inner aggregate: group by the anchor, one count
+    const Expr *ge = inner->groups.size() == 1 ? strip_value_preserving_casts(&inner->groups[0]) : nullptr;
+    BaseCol gk;
+    if (!ge || ge->kind != PG_TK_COL || ge->idx < 0 || ge->idx >= (int)J.outs.size() || J.outs[(size_t)ge->idx].first != 0 || !resolve(J, ge->idx, &gk) ||
+        gk.slot != pk.slot || gk.col != pk.col)
+        PG_FAIL(PG_EUNSUPPORTED, "the group key is not the anchor (the preserved side's join key) alone");
+    if (inner->aggs.size() != 1 || inner->aggs[0].fn != PG_AGG_COUNT || inner->aggs[0].ltype != PG_LT_HUGEINT)
+        PG_FAIL(PG_EUNSUPPORTED, "the per-group aggregate is not exactly one count");
+    if (!inner->aggs[0].star) {
+        const Expr *ae = strip_value_preserving_casts(&inner->aggs[0].arg);
+        BaseCol ak;
+        if (ae->kind != PG_TK_COL || ae->idx < 0 || ae->idx >= (int)J.outs.size() || !resolve(J, ae->idx, &ak))
+            PG_FAIL(PG_EUNSUPPORTED, "the count argument is not a column");
+        if (J.outs[(size_t)ae->idx].first == 1) {
+            p->arg_col = ak.col;
+            p->null_if_empty = true;
+        } else if (at->cols[(size_t)ak.col].any_nulls()) {
+            PG_FAIL(PG_EUNSUPPORTED, "count over a nullable preserved-side column");
+        }
+    }
+    for (auto &o : inner->outs)
+        if (o != std::make_pair(0, 0) && o != std::make_pair(1, 0)) PG_FAIL(PG_EUNSUPPORTED, "bad output of the per-group aggregate");
+    p->outs = inner->outs;
+    if (p->outer) {
+        const Expr *oe = root.groups.size() == 1 ? strip_value_preserving_casts(&root.groups[0]) : nullptr;
+        if (!oe || oe->kind != PG_TK_COL || oe->idx < 0 || oe->idx >= (int)inner->outs.size() || inner->outs[(size_t)oe->idx] != std::make_pair(1, 0))
+            PG_FAIL(PG_EUNSUPPORTED, "the outer aggregate is not grouped by the per-group count alone");
+        if (root.aggs.size() != 1 || root.aggs[0].fn != PG_AGG_COUNT || !root.aggs[0].star || root.aggs[0].ltype != PG_LT_HUGEINT)
+            PG_FAIL(PG_EUNSUPPORTED, "the outer aggregate is not count(*)");
+        for (auto &o : root.outs)
+            if (o != std::make_pair(0, 0) && o != std::make_pair(1, 0)) PG_FAIL(PG_EUNSUPPORTED, "bad output of the outer aggregate");
+        p->outs = root.outs;
+    }
+    if (bt->nrows >= ((i64)1 << 32)) PG_FAIL(PG_EUNSUPPORTED, "the build side has 2^32 rows or more (the per-row counts are 32-bit)");
+    if (at->nrows >= ((i64)1 << 32)) PG_FAIL(PG_EUNSUPPORTED, "the preserved side has 2^32 rows or more");
+    {
+        LowerCtx cx;
+        cx.table = bt;
+        cx.allow_nulls = true;
+        std::vector<Expr> fl = bs->filters;
+        for (auto &f : bf) fl.push_back(f);
+        if (!lower_filters(cx, fl, p->build_ranges)) PG_FAIL(PG_EUNSUPPORTED, "build-side filter not off-loadable: %s", cx.why.c_str());
+    }
+    int stage = -1;
+    PG_TRY(add_build_stage(&p->jp, J.children[0], pe->idx, &stage));
+    p->jp.stages[(size_t)stage]->payload_needed = true;
+    p->anchor_col = pk.col;
+    p->build_slot = bk.slot;
+    p->build_key_col = bk.col;
+    p->big_cap = bt->nrows / LC_HBINS + 1;
+    std::vector<std::string> likes;
+    PG_TRY(p->fill(p->fa, p->jp.stages[(size_t)stage]->ranges, pk.slot, nullptr));
+    PG_TRY(p->fill(p->fb, p->build_ranges, bk.slot, &likes));
+    PG_TRY(p->jp.d_counters.alloc(128));
+    // the pass reads the build side's key, count argument, predicate columns and string bytes + offsets once
+    auto colbytes = [&](const pg_table *t, int col) -> i64 {
+        const Column &cc = t->cols[(size_t)col];
+        if (cc.type == PG_T_VARCHAR) return (i64)cc.h_bytes.size() + (t->nrows + 1) * 8;
+        return t->nrows * cc.phys_width();
+    };
+    std::vector<int> read{bk.col};
+    if (p->arg_col >= 0) read.push_back(p->arg_col);
+    for (auto &r : p->build_ranges) read.push_back(r.col);
+    std::sort(read.begin(), read.end());
+    read.erase(std::unique(read.begin(), read.end()), read.end());
+    for (int col : read) p->main_bytes += colbytes(bt, col);
+    p->algorithmic_bytes = p->main_bytes + colbytes(at, pk.col);
+    std::string pass;
+    if (!p->fb.npred && likes.empty()) pass = " every row";
+    if (p->fb.npred) pass += " ranges=" + std::to_string(p->fb.npred);
+    for (size_t i = 0; i < likes.size(); i++) pass += (i ? "," : " like=") + likes[i];
+    p->explain = "left-join count: groups=rows of " + at->name + "; " + bt->name + " pass" + pass + "; kernel=left_count_kernel+" +
+                 (p->outer ? "count_hist_kernel" : "left_compact_kernel");
     *out = std::move(p);
     return PG_OK;
 }

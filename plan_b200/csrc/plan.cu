@@ -21,6 +21,7 @@ Pipeline::~Pipeline() {}
 int build_scan_agg(pg_plan *plan, const Node &agg, const Node &scan, std::unique_ptr<Pipeline> *out);
 int build_join_agg(pg_plan *plan, const Node &agg, const Node &join, std::unique_ptr<Pipeline> *out, bool nested = false);
 int build_rows(pg_plan *plan, std::unique_ptr<Pipeline> *out, const Node *aggn = nullptr);      // rows.cu: row-emitting Scan / Filter / Project / Join; aggn: aggregate over the joined rows
+int build_left_count(pg_plan *plan, const Node &root, std::unique_ptr<Pipeline> *out);            // join.cu: per-row counts of a LEFT join [+ Agg over them]
 
 static const Node *skip_filters(const Node *n, std::vector<Expr> *extra)
 {
@@ -238,7 +239,19 @@ static int build_pipeline(pg_plan *plan)
         // a LEFT join ...): one join of two scans can still run as row programs over the joined rows (rows.cu)
         plan->pipe.reset();
         s = build_rows(plan, &plan->pipe, &root);
-        if (s == PG_EUNSUPPORTED) PG_FAIL(PG_EUNSUPPORTED, "%s; expression-driven join aggregate: %s", why.c_str(), std::string(get_error()).c_str());
+        if (s != PG_EUNSUPPORTED) return s;
+        const std::string why2 = get_error();
+        // a LEFT join counted per preserved row (TPC-H Q13's inner aggregate)
+        plan->pipe.reset();
+        s = build_left_count(plan, root, &plan->pipe);
+        if (s == PG_EUNSUPPORTED)
+            PG_FAIL(PG_EUNSUPPORTED, "%s; expression-driven join aggregate: %s; left-join count: %s", why.c_str(), why2.c_str(), std::string(get_error()).c_str());
+        return s;
+    }
+    if (child->op == PG_OP_AGG) {
+        // an aggregate over an aggregate: only the distribution of per-row LEFT-join counts (TPC-H Q13)
+        const int s = build_left_count(plan, root, &plan->pipe);
+        if (s == PG_EUNSUPPORTED) PG_FAIL(PG_EUNSUPPORTED, "unsupported aggregate input (op %d); left-join count: %s", child->op, std::string(get_error()).c_str());
         return s;
     }
     PG_FAIL(PG_EUNSUPPORTED, "unsupported aggregate input (op %d)", child->op);

@@ -222,6 +222,30 @@ inline bool like_is_contains(const std::string &pat, std::string *lit)
     return true;
 }
 
+// `%s1%s2%...%sk%`: a leading and a trailing '%', runs of '%' taken as one, 1 <= k <= LIKE_MAXSEG segments of 1..8 bytes
+// without '_'.  Such a pattern matches exactly when the segments occur in order without overlapping, and the leftmost
+// occurrence of each segment after the end of the previous one decides: the device searches one segment at a time
+// with the word-at-a-time search (kinds GEN_LIKE_WORDS / GEN_NOTLIKE_WORDS, leftcount.cuh).
+constexpr int LIKE_MAXSEG = 4;
+inline bool like_segments(const std::string &pat, std::vector<std::string> *segs)
+{
+    segs->clear();
+    if (pat.size() < 3 || pat.front() != '%' || pat.back() != '%') return false;
+    std::vector<std::string> out;
+    std::string cur;
+    for (char ch : pat) {
+        if (ch == '_') return false;
+        if (ch != '%') { cur += ch; continue; }
+        if (cur.empty()) continue;
+        if (cur.size() > 8 || (int)out.size() == LIKE_MAXSEG) return false;
+        out.push_back(cur);
+        cur.clear();
+    }
+    if (out.empty()) return false;
+    segs->swap(out);
+    return true;
+}
+
 // The reference's LIKE matcher restated (wildcardMatch, function_operator_boolean.go:336-377): byte-wise,
 // '%' matches any run (greedy with backtracking to the last '%'), '_' any single byte.
 inline bool wildcard_match(const char *pat, size_t plen, const char *tgt, size_t tlen)

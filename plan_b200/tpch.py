@@ -742,17 +742,20 @@ Q13_CUSTOMER = [("c_custkey", L.PG_T_INT32, 0, 0, None)]
 Q13_ORDERS = [("o_orderkey", L.PG_T_INT64, 0, 0, None), ("o_custkey", L.PG_T_INT32, 0, 0, None), ("o_comment", L.PG_T_VARCHAR, 79, 0, None)]
 
 
-def q13_plan(pattern="%pending%accounts%"):
+def q13_plan(pattern="%pending%accounts%", outer=True):
     """cases/tpch/query/q13.sql:  Agg(group by c_count; count(*)) <- Agg(group by c_custkey; count(o_orderkey))
       <- LeftJoin(c_custkey = o_custkey) <- { Scan(customer), Scan(orders; o_comment not like pattern) }.
     The ON-clause predicate on orders alone filters the build side; customers without a surviving order keep one NULL-padded row,
-    over which count(o_orderkey) is NULL in the reference (CountOp.Finalize) -- q13.txt's first row.  Plan tree only (see Q5 / Q7 / Q8)."""
+    over which count(o_orderkey) is NULL in the reference (CountOp.Finalize) -- q13.txt's first row.  The GPU runs it as a grouped
+    LEFT-join count (join.cu build_left_count).  outer=False: the inner aggregate alone, (c_custkey, c_count) per customer."""
     B, V, I, BI, H = K.LType(K.LTID_BOOLEAN), K.VarcharType(), K.IntegerType(), K.BigintType(), K.HugeintType()
     cust = PhysicalOperator(POT_Scan, Info=ScanOpInfo("customer"))
     orders = PhysicalOperator(POT_Scan, Info=ScanOpInfo("orders"), Filters=[func("not like", B, col(0, 2, V), const(pattern, V))])
     j = PhysicalOperator(POT_Join, Children=[cust, orders], Outputs=[col(0, 0, I), col(1, 0, BI)],
                          Info=JoinOpInfo(JOIN_LEFT, [func("=", B, col(0, 0, I), col(1, 1, I))]))
     per_cust = PhysicalOperator(POT_Agg, Outputs=[col(0, 0, I), col(1, 0, H)], Children=[j], Info=AggOpInfo([func("count", H, col(0, 1, BI))], [col(0, 0, I)]))
+    if not outer:
+        return per_cust
     return PhysicalOperator(POT_Agg, Outputs=[col(0, 0, H), col(1, 0, H)], Children=[per_cust], Info=AggOpInfo([func("count", H)], [col(0, 1, H)]))
 
 
